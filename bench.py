@@ -2,8 +2,11 @@
 """Headline benchmark: FNO-family train step (fwd + MSE + bwd + Adam) samples/s on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|cfg1|cfg3]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); rank 0 prints ONE JSON line.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last step handed its caller as DIR/<name>.npy (see
+dump_outputs); inputs and weights are seeded, so two builds of the project can be compared output for output.
 
 Workload at N=1 (BASELINE.json configs[1], the config the metric's target is quoted on):
 TFNO2D (Tucker rank 0.8) on 64x64 synthetic fields, 1 -> 1 channels, width 64, 16 modes, 4 layers,
@@ -57,6 +60,42 @@ WORKLOADS = {
 def log(msg):
     sys.stderr.write(f"[bench {time.strftime('%H:%M:%S')}] {msg}\n")
     sys.stderr.flush()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, arrays, limit=DUMP_BYTES):
+    """Write ``arrays`` (name -> tensor; None entries are skipped) as ``path/<name>.npy`` in float32 (float64 stays
+    float64), at most ``limit`` bytes of files in all.  Arrays are taken smallest first and each is written whole when
+    it fits an equal share of what is left.  One that does not is written as a flat 1-D sample: its elements at the
+    distinct flat indices among that many draws from a fixed seed (with replacement, so somewhat fewer than the share),
+    in index order, so the same workload gives the same sample on every run; neither the shape nor the indices are
+    written."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    items = sorted(((k, v) for k, v in arrays.items() if v is not None), key=lambda kv: kv[1].numel())
+    left = limit
+    for i, (name, t) in enumerate(items):
+        t = t.detach()
+        t = t if t.dtype == torch.float64 else t.float()
+        share = left // (len(items) - i) - 128                     # 128: the .npy header
+        if t.numel() * t.element_size() > share:
+            idx = torch.randint(t.numel(), (max(share, 0) // t.element_size(),), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[idx.unique().to(t.device)]            # sorted, distinct
+        fn = os.path.join(path, name + ".npy")
+        np.save(fn, t.cpu().numpy())
+        left -= os.path.getsize(fn)
+
+
+def _train_step_outputs(out, loss, model):
+    """What one train step hands its caller: the model output, the loss, every gradient and every updated parameter."""
+    d = {"output": out, "loss": loss}
+    for k, p in model.named_parameters():
+        d["param." + k] = p
+        d["grad." + k] = p.grad
+    return d
 
 
 def build_model(wl, seed=1234):
@@ -510,6 +549,9 @@ def run_afno(args, wl, rank, world, local_rank):
     full = wl["kind"] == "afnonet"
     B, H, W, C = wl["batch"], wl["H"], wl["W"], wl["embed"]
     g = torch.Generator().manual_seed(1234 + rank)
+    # output of the latest step (inside the graph: its static output), detached: holding its autograd graph would carry
+    # the parameters' AccumulateGrad nodes of an eager step, bound to the eager stream, into the graph capture
+    last = {}
     if full:
         model = _build_afnonet(pkg, wl).to(dev)
         host = [torch.randn(B, 1, 4, H, W, generator=g).pin_memory(), torch.randn(B, 2, 1, H, W, generator=g).pin_memory(),
@@ -518,6 +560,7 @@ def run_afno(args, wl, rank, world, local_rank):
 
         def fwd_loss():
             out = model(constants=dv[0], prescribed=dv[1], prognostic=dv[2])      # [B, 1, 8, H, W]
+            last["out"] = out.detach()
             return torch.nn.functional.mse_loss(out, dv[2][:, 1:])
     else:
         model = torch.nn.Sequential(*[pkg.AFNO2D(C, num_blocks=wl["nb"]) for _ in range(wl["depth"])]).to(dev)
@@ -525,7 +568,9 @@ def run_afno(args, wl, rank, world, local_rank):
         dv = [t.to(dev) for t in host]
 
         def fwd_loss():
-            return torch.nn.functional.mse_loss(model(dv[0]), dv[1])
+            out = model(dv[0])
+            last["out"] = out.detach()
+            return torch.nn.functional.mse_loss(out, dv[1])
     params = list(model.parameters())
     opt = torch.optim.Adam(params, lr=1e-3, fused=True, capturable=True)
     sync = GradSync(params, world) if world > 1 else None
@@ -581,6 +626,8 @@ def run_afno(args, wl, rank, world, local_rank):
         hloss.copy_(loss_buf, non_blocking=True)
         torch.cuda.current_stream().synchronize()
     t_e2e, _ = _timed(step_e2e, args.steps, 3, world, local_rank, dist)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, _train_step_outputs(last["out"], loss_buf, model))
     tt = torch.tensor([t_dev, t_e2e], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -668,6 +715,8 @@ def run_rollout(args, wl, rank, world, local_rank):
         hlast.copy_(out[:, -1], non_blocking=True)
         torch.cuda.current_stream().synchronize()
     t_e2e, _ = _timed(step_e2e, args.steps, 1, world, local_rank, dist)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"output": out})          # [B, R, C, H, W] frames of the last rollout
     tt = torch.tensor([t_dev, t_e2e], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -725,9 +774,13 @@ def run_b200(args, wl, rank, world, local_rank):
     x, y = hx.to(dev), hy.to(dev)
     loss_buf = torch.zeros((), device=dev)
     hloss = torch.zeros((), pin_memory=True)
+    # output of the latest step (inside the graph: its static output), detached: holding its autograd graph would carry
+    # the parameters' AccumulateGrad nodes of an eager step, bound to the eager stream, into the graph capture
+    last = {}
 
     def fwd_bwd():
         out = model(x)
+        last["out"] = out.detach()
         loss = torch.nn.functional.mse_loss(out, y)
         loss.backward()
         loss_buf.copy_(loss.detach())
@@ -844,6 +897,8 @@ def run_b200(args, wl, rank, world, local_rank):
     e1.record()
     barrier()
     t_e2e = e0.elapsed_time(e1) * 1e-3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, _train_step_outputs(last["out"], loss_buf, model))
 
     tt = torch.tensor([t_dev, t_e2e], device=dev, dtype=torch.float64)
     if world > 1:
@@ -930,10 +985,16 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--ddp-sum", action="store_true", help="gradient all-reduce as SUM + scale instead of ReduceOp.AVG")
     ap.add_argument("--skip-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last step as DIR/<name>.npy (b200 arm)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.steps is None:
         args.steps = 20 if (args.impl == "reference" or args.workload in ("cfg3", "cfg5")) else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

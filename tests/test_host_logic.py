@@ -105,12 +105,17 @@ def test_mode_block_matches_oracle():
         assert fno_mode_block(H, 64, (n, 7)) == (lo - H // 2, My, 7)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not present on this box")
+# root of a checkout of amazon-science/dlwp-benchmark, the project whose wrappers the shim serves (not vendored here)
+REFERENCE = os.environ.get("DLWP_BENCHMARK_REFERENCE", "")
+
+
+@pytest.mark.skipif(not REFERENCE or not os.path.isdir(os.path.join(REFERENCE, "src")),
+                    reason="set DLWP_BENCHMARK_REFERENCE to a checkout of amazon-science/dlwp-benchmark")
 def test_reference_wrappers_import_on_the_shim():
     """The UNMODIFIED reference wrapper modules import and construct on top of the shim."""
     import importlib.util
     pkg.install_neuralop_shim(force=True)
-    path = "/root/reference/src/nsbench/models/fno/fno.py"
+    path = os.path.join(REFERENCE, "src", "nsbench", "models", "fno", "fno.py")
     spec = importlib.util.spec_from_file_location("_ref_ns_fno", path)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
@@ -121,6 +126,34 @@ def test_reference_wrappers_import_on_the_shim():
     t = mod.TFNO2DModule(n_modes=[12, 12], in_channels=1, hidden_channels=8, lifting_channels=16,
                          projection_channels=16, out_channels=1, n_layers=1, rank=0.5, context_size=2)
     assert "fno.fno_blocks.convs.weight.0.tensor" in t.state_dict()     # dense: the reference's own quirk
+
+
+def test_neuralop_imports_resolve_to_the_shim():
+    """The reference wrappers do `from neuralop.models import FNO, TFNO` (src/nsbench/models/fno/fno.py:7): with the
+    shim installed those names, and neuralop's SpectralConv, are this package's classes; the shim refuses to shadow a
+    real neuralop unless forced."""
+    import sys
+    import types
+    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] == "neuralop"}
+    try:
+        for k in saved:
+            del sys.modules[k]
+        pkg.install_neuralop_shim()
+        from neuralop.models import FNO, TFNO
+        from neuralop.layers.spectral_convolution import SpectralConv
+        assert (FNO, TFNO, SpectralConv) == (pkg.FNO, pkg.TFNO, pkg.SpectralConv)
+        w = FNO(n_modes=[12, 12], in_channels=1, hidden_channels=8, lifting_channels=16, projection_channels=16,
+                out_channels=1, n_layers=1, rank=0.5)
+        assert "fno_blocks.convs.weight.0.tensor" in w.state_dict()        # FNO(..., rank=rank) stays dense
+        pkg.install_neuralop_shim()                                         # installing over the shim is fine
+        sys.modules["neuralop"] = types.ModuleType("neuralop")               # a real neuralop imported first
+        with pytest.raises(RuntimeError):
+            pkg.install_neuralop_shim()
+        assert pkg.install_neuralop_shim(force=True).models.FNO is pkg.FNO
+    finally:
+        for k in [k for k in sys.modules if k.split(".")[0] == "neuralop"]:
+            del sys.modules[k]
+        sys.modules.update(saved)
 
 
 def test_sequence_forward_is_the_reference_loop():
@@ -160,3 +193,28 @@ def test_bench_reads_traffic_from_the_committed_capture():
     # the skip-conv weight gradient reads g and x once each (2 x 67 MB), not the 336 MB of the projection-head launch
     assert bench._ncu_traffic("tc_wgrad_kernel<3, 0>", 8 * 64 * 64 * 64 * 64) < 200e6
     assert bench._cpu_sample(bench.WORKLOADS["cfg2"]) == 64 and bench._cpu_sample(bench.WORKLOADS["cfg3"]) == 2
+
+
+def test_bench_dump_outputs_stays_within_its_limit(tmp_path):
+    """bench.py --dump-outputs: one .npy per array, float32 (float64 kept), whole while the arrays fit the limit;
+    beyond it the largest array becomes a flat sample at distinct indices, the same ones on every call."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(0)
+    arrays = {"loss": torch.tensor(0.25), "w": torch.randn(3, 4, dtype=torch.float64, generator=g),
+              "h": torch.randn(64, dtype=torch.float16, generator=g), "none": None,
+              "big": torch.randn(50_000, generator=g)}
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    got = {f[:-4]: np.load(tmp_path / "whole" / f) for f in os.listdir(tmp_path / "whole")}
+    assert set(got) == {"loss", "w", "h", "big"}
+    assert got["loss"].dtype == np.float32 and got["loss"].shape == () and got["loss"] == 0.25
+    assert got["w"].dtype == np.float64 and np.array_equal(got["w"], arrays["w"].numpy())
+    assert got["h"].dtype == np.float32 and np.array_equal(got["h"], arrays["h"].float().numpy())
+    assert np.array_equal(got["big"], arrays["big"].numpy())
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, limit=40_000)
+        assert sum(os.path.getsize(tmp_path / run / f) for f in os.listdir(tmp_path / run)) <= 40_000
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert 5_000 < a.size < 10_000 and np.array_equal(a, b) and np.isin(a, got["big"]).all()
+    assert np.unique(a).size == a.size                     # distinct indices (the values are distinct normals)
+    assert np.array_equal(np.load(tmp_path / "a" / "w.npy"), got["w"])

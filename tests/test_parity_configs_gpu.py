@@ -93,6 +93,50 @@ def test_cfg2_full_tfno_model_fwd_loss_all_grads_and_graph_replay():
     _check_grads(m, go, 2e-5)
 
 
+@pytest.mark.parametrize("workload", ["cfg2", "cfg4"])
+def test_bench_dump_outputs_hold_the_last_captured_step(tmp_path, workload):
+    """bench.py --dump-outputs through the replayed CUDA graph (FNO arm cfg2, AFNO arm cfg4): the dumped output and
+    loss belong to the same step (MSE of the output against the seeded target == the loss; for cfg2 also == the loss
+    the step read back), every parameter and gradient is there in float32, and a second run dumps the same arrays."""
+    import json
+    import subprocess
+    import numpy as np
+    wl = bench.WORKLOADS[workload]
+    runs = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", workload, "--steps", "2",
+                            "--warmup", "3", "--skip-cpu", "--skip-roofline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 2 and (line.get("run") or line["config"])["cuda_graph"]
+        runs.append({f[:-4]: np.load(d / f) for f in os.listdir(d)})
+    got = runs[0]
+    g = torch.Generator().manual_seed(1234)
+    if workload == "cfg2":
+        m = bench.build_model(wl)
+        torch.randn(wl["batch"], 1, wl["H"], wl["W"], generator=g)                            # x
+        target = torch.randn(wl["batch"], 1, wl["H"], wl["W"], generator=g)
+        assert float(got["loss"]) == line["e2e"]["last_loss"]
+    else:
+        m = bench._build_afnonet(pkg, wl)
+        B, H, W = wl["batch"], wl["H"], wl["W"]
+        torch.randn(B, 1, 4, H, W, generator=g), torch.randn(B, 2, 1, H, W, generator=g)      # constants, prescribed
+        target = torch.randn(B, 2, wl["cout"], H, W, generator=g)[:, 1:]
+    assert got["output"].shape == tuple(target.shape)
+    loss = F.mse_loss(torch.from_numpy(got["output"]).double(), target.double()).item()
+    assert abs(loss - float(got["loss"])) / float(got["loss"]) < 1e-5
+    names = {k for k, _ in m.named_parameters()}
+    assert {k[6:] for k in got if k.startswith("param.")} == names
+    unused = {"norm.weight", "norm.bias"} if workload == "cfg4" else set()       # AFNONet's final norm: no gradient
+    assert {k[5:] for k in got if k.startswith("grad.")} == names - unused
+    assert all(a.dtype == np.float32 and np.isfinite(a).all() for a in got.values())
+    assert set(runs[1]) == set(got)
+    for k, a in got.items():
+        assert np.linalg.norm(runs[1][k] - a) <= 1e-6 * np.linalg.norm(a), k
+
+
 def test_dlwpbench_shape_whole_model_13_to_8_channels_32x64():
     """dlwpbench FNO (src/dlwpbench/configs/model/fno.yaml: 4 + 9*1 = 13 in, 8 out, 32x64 grid, 12 modes,
     width 32, lifting / projection 256): no fused head (n_out != 1), small-M lifting path."""
